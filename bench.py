@@ -54,7 +54,15 @@ def parse_args():
                     help="c2 (default, the contract line): BASELINE config 2 join; q3 / c5: BASELINE configs 4 / 5 pipelines")
     ap.add_argument("--slabs", type=int, default=int(os.environ.get("GSQL_BENCH_SLABS", "1")),
                     help="slabs of the pushed side (N > 1): slab k is consumed while slab k+1 crosses NVLink; 1 measured best at N = 2..8 (r02)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's output columns to DIR/<workload>_<name>.npy (float64, a seeded sample "
+                         "of at most 2^20 rows per table) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm returns row counts only)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks sampler
@@ -400,6 +408,9 @@ def run_ours(args):
     n_out = state["out_rows"]
     parity = verify_join_checksum(torch, dist, synth, dev, world, rank, nb, npr, probe, out_cols, n_out)
     assert parity["match"], f"join output checksum mismatch: {parity}"
+    if args.dump_outputs:
+        names = ["probe_key", "probe_p1", "probe_p2", "build_key", "build_b1", "build_b2"]
+        dump_outputs(args.dump_outputs, "c2", [(nm, d[:n_out], None) for nm, (d, _) in zip(names, out_cols)], 3, rank, world)
 
     # ---- roofline of the dominant kernel(s): the probe phase
     probe_kernels = [k for k in prof if "probe" in k or k == "join_scan"]
@@ -526,6 +537,48 @@ def verify_join_checksum(torch, dist, synth, dev, world, rank, nb, npr, probe, o
             "what": "sum over all output rows of mix64(probe.key,p1,p2,b1,b2), all ranks, vs the same sum derived from the inputs"}
 
 
+DUMP_ROWS = 1 << 20   # rows written per output table and run: at most 6 float64 columns -> 48 MB per dump
+
+
+def dump_outputs(out_dir, workload, cols, nkey, rank, world, chunk=1 << 26):
+    """--dump-outputs: write `cols` ([(name, device values, device nulls | None)], one output table of the last step) as
+    out_dir/<workload>_<name>.npy, float64 with NaN for NULL, plus <workload>_rows.npy = [total output rows].
+
+    Row order out of a hash join / group-by is unspecified, so the dump must not depend on it: when the table has more
+    than DUMP_ROWS rows, a row is kept when a seeded hash of its first `nkey` columns (the columns that identify it: probe
+    row, group key) falls under a threshold, and the kept rows are sorted on all columns.  Two builds that produce the
+    same rows therefore write the same arrays.  Every integer these workloads produce is below 2^53, so float64 holds it
+    exactly.  With N ranks each rank writes its own share (suffix .rank<r>), DUMP_ROWS / N rows each."""
+    import numpy as np
+    import torch
+    from galaxysql_b200 import synth
+    cap = DUMP_ROWS // world
+    n = int(cols[0][1].numel())
+    threshold = None if n <= cap else int(0.9 * cap / n * (1 << 53))   # ~0.9 * cap rows kept; truncation below never bites
+    parts = [[] for _ in cols]
+    for lo in range(0, n, chunk):
+        hi = min(n, lo + chunk)
+        f64 = []
+        for _, d, nl in cols:
+            v = d[lo:hi].to(torch.float64)
+            f64.append(v if nl is None else torch.where(nl[lo:hi].bool(), float("nan"), v))
+        if threshold is not None:
+            h = torch.full((hi - lo,), synth.SEED, dtype=torch.int64, device=f64[0].device)
+            for v in f64[:nkey]:
+                h = synth.splitmix64_t(h ^ v.view(torch.int64))
+            keep = synth._lsr(h, 11) < threshold
+            f64 = [v[keep] for v in f64]
+        for p, v in zip(parts, f64):
+            p.append(v.cpu().numpy())
+    arrays = [np.concatenate(p) if p else np.zeros(0) for p in parts]
+    order = np.lexsort(arrays[::-1])[:cap]
+    suffix = "" if world == 1 else f".rank{rank}"
+    os.makedirs(out_dir, exist_ok=True)
+    for (name, _, _), a in zip(cols, arrays):
+        np.save(os.path.join(out_dir, f"{workload}_{name}{suffix}.npy"), a[order])
+    np.save(os.path.join(out_dir, f"{workload}_rows{suffix}.npy"), np.array([n], dtype=np.float64))
+
+
 def _timed_agg(ctx, make, feed, reps=3):
     """Best wall time of consume+finish over `reps` fresh handles (after one warm-up), and the kernel times of that run."""
     import time as _t
@@ -609,12 +662,13 @@ def run_aux_agg_c1(ctx, api, N, synth, dev, scale, peak_gbs):
 
 # ------------------------------------------------------------------------------------------------ q3 / c5 pipelines
 def run_pipeline_workload(args, ctx, stream, world, rank, local_rank, dev):
-    line = measure_pipeline(args, args.workload, args.steps, args.warmup, ctx, stream, world, rank, local_rank, dev, with_clocks=True)
+    line = measure_pipeline(args, args.workload, args.steps, args.warmup, ctx, stream, world, rank, local_rank, dev, with_clocks=True,
+                            dump_dir=args.dump_outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
 
 
-def measure_pipeline(args, workload, steps, warmup, ctx, stream, world, rank, local_rank, dev, with_clocks=False):
+def measure_pipeline(args, workload, steps, warmup, ctx, stream, world, rank, local_rank, dev, with_clocks=False, dump_dir=None):
     """workload q3: BASELINE config 4 (TPC-H Q3, SF300 over 8 GPUs = SF37.5 per GPU, weak scaling);
     --workload c5: BASELINE config 5 (GROUP BY k, SUM(double): 500 M rows and 6.25 M keys per GPU).  One step = the whole
     pipeline of galaxysql_b200/pipelines.py over device-resident tables; value = input rows of all ranks / max step time."""
@@ -745,6 +799,9 @@ def measure_pipeline(args, workload, steps, warmup, ctx, stream, world, rank, lo
                   "groups": int(got[2]), "what": "sum of SUM(v) and of COUNT(*) over all groups vs the column totals; groups <= distinct keys"}
         stats = {"mode": agg.mode}
     assert parity["match"], parity
+    if dump_dir:
+        names = ["l_orderkey", "o_orderdate", "o_shippriority", "revenue"] if workload == "q3" else ["k", "sum_v", "count_star"]
+        dump_outputs(dump_dir, workload, [(nm, d, nl) for nm, (d, nl) in zip(names, out)], 3 if workload == "q3" else 1, rank, world)
     (q3 if workload == "q3" else agg).close()
     value = rows_in * world / (ms_step / 1e3)
     return {"metric": METRIC, "value": value, "unit": "rows/s", "n_gpus": world, "steps": steps, "warmup": warmup,
